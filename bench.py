@@ -2,6 +2,7 @@
 """bench.py -- point-clouds/sec of the SECOND LiDAR-inference hot path on B200 (BASELINE.json metric).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b2second|reference] [--config car.fhd]
+                  [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one pass of the hot path (voxelize -> sparse middle -> BEV -> RPN -> decode/NMS) over one batch
@@ -24,6 +25,9 @@ Prints ONE JSON line (rank 0):
             config, each with its stage split and RPN tensor rate
   cpu_baseline  the same network through the CPU oracle (`port`: C voxelizer/NMS + torch-CPU sparse conv/RPN)
             on a bounded sample of the same workload, host cores of this box
+--dump-outputs DIR: after the timed steps, the detections of the last timed step of each timed path (resident:
+  engine.infer, e2e: net(example)) go to DIR as float32 .npy files, so that two builds can be compared output for
+  output (same arguments -> same seeded clouds and weights).
 --impl reference: the reference arm = the reference's CPU implementation of the path.  spconv 1.x is not
   in the reference tree and cannot be installed (no network), so this is the oracle port timed with all host
   threads (DESIGN.md "reference arm").
@@ -64,6 +68,8 @@ def parse():
                     help="sparse-conv inner product: tc = tcgen05 3xF16 split, fma = fp32 FMA tiles")
     ap.add_argument("--rpn", default="auto", choices=["auto", "tc", "cudnn"],
                     help="RPN implementation: tc = hand-written tcgen05 3xF16 implicit GEMM, cudnn = torch fp32")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the detections of the last timed step of each timed path to DIR/<path>_<field>.npy")
     return ap.parse_args()
 
 
@@ -182,6 +188,22 @@ def run_reference_arm(args):
             "e2e": {"value": value, "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
             "gpu_launches": 0}
     print(json.dumps(line), flush=True)
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_detections(out_dir, path, dets):
+    """one step's per-frame detection dicts (the reference's list of dicts) as float32 arrays: the rows of all frames
+    concatenated in frame order, <path>_frame.npy holding each row's frame index."""
+    arrays = {f: np.concatenate([np.asarray(d[f], dtype=np.float32) for d in dets])
+              for f in ("box3d_lidar", "scores", "label_preds")}
+    arrays["frame"] = np.repeat(np.arange(len(dets)), [len(d["scores"]) for d in dets]).astype(np.float32)
+    if sum(a.nbytes for a in arrays.values()) > DUMP_LIMIT_BYTES:
+        raise SystemExit("bench.py: --dump-outputs would write more than %d bytes" % DUMP_LIMIT_BYTES)
+    os.makedirs(out_dir, exist_ok=True)
+    for f, a in arrays.items():
+        np.save(os.path.join(out_dir, "%s_%s.npy" % (path, f)), a)
 
 
 # ------------------------------------------------------------------------------------------------ clocks
@@ -360,10 +382,12 @@ def run_gpu_arm(args):
         if gather is not None:
             gather.gather_records(eng.det_record)
 
+    last = {}
+
     def step_e2e(i):
         # pinned host clouds in, host tensors out: H2D of the points, the graph, the all-gather (N > 1) and ONE D2H
         # of the detection records all happen inside this call
-        net({"points": host[i % n_sets], "anchors": anchors})
+        last["e2e"] = net({"points": host[i % n_sets], "anchors": anchors})
 
     warm = max(args.warmup, 3)
     sampler = ClockSampler(local)
@@ -380,7 +404,12 @@ def run_gpu_arm(args):
         torch.cuda.profiler.stop()
         return
     ms_res = _timed(step_resident, args.steps, warm, flush, world, dev)
+    if args.dump_outputs:      # the detection records the last resident step left on the device, before e2e reuses them
+        last["resident"] = eng.detections()
     ms_e2e = _timed(step_e2e, args.steps, warm, flush, world, dev)
+    if args.dump_outputs and rank == 0:
+        for path in ("resident", "e2e"):
+            dump_detections(args.dump_outputs, path, last[path])
     clocks = sampler.stop() if rank == 0 else None
     eng.check_status()
     frames = world * B * args.steps

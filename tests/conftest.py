@@ -47,26 +47,3 @@ def out_dir():
     os.makedirs(d, exist_ok=True)
     return d
 
-
-@pytest.fixture(scope="module")
-def ref_env():
-    # the reference imports its plugin by the name `spconv`: make that name the CPU oracle for this module's
-    # tests (other test modules in the same process use the CUDA drop-in under that name), then restore
-    saved = {k: v for k, v in sys.modules.items() if k == "spconv" or k.startswith("spconv.")}
-    for k in saved:
-        del sys.modules[k]
-    saved_path = list(sys.path)
-    from b2second import loader as _loader
-    sys.path[:] = [p for p in sys.path if os.path.abspath(p) != os.path.abspath(_loader.PRODUCT_DIR)] + \
-        [_loader.PRODUCT_DIR]
-    from b2second import loader, refcompat
-    refcompat.install(loader.ORACLE_DIR)
-    import spconv
-    assert getattr(spconv, "__oracle__", False)
-    yield spconv
-    for k in [k for k in sys.modules if k == "spconv" or k.startswith("spconv.")]:
-        del sys.modules[k]
-    sys.modules.update(saved)
-    sys.path[:] = saved_path
-
-

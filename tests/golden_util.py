@@ -1,6 +1,8 @@
 """helpers shared by the golden-fixture tests (CPU oracle path and GPU product path)."""
+import dataclasses
 import glob
 import hashlib
+import json
 import os
 
 import numpy as np
@@ -8,6 +10,66 @@ import numpy as np
 from b2second import config, synth
 
 GOLDEN_DIR = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+
+
+def digest(a):
+    """dtype, shape and sha1 of a tensor or array: equal digests <=> equal arrays (bit for bit)."""
+    if hasattr(a, "detach"):
+        a = a.detach().cpu().numpy()
+    a = np.ascontiguousarray(a)
+    return {"dtype": a.dtype.name, "shape": list(a.shape), "sha1": hashlib.sha1(a.tobytes()).hexdigest()}
+
+
+def jsonable(x):
+    """the plain-JSON form of a config, spec signature or launch plan; tensors and arrays become digests, so
+    jsonable(a) == jsonable(b) <=> a == b field by field (torch.equal for tensors)."""
+    if hasattr(x, "detach") or isinstance(x, np.ndarray):
+        return digest(x)
+    if dataclasses.is_dataclass(x) and not isinstance(x, type):
+        return jsonable(dataclasses.asdict(x))
+    if isinstance(x, dict):
+        return {str(k): jsonable(v) for k, v in x.items()}
+    if isinstance(x, (list, tuple)):
+        return [jsonable(v) for v in x]
+    if isinstance(x, np.generic):
+        return x.item()
+    if x is None or isinstance(x, (bool, int, float, str)):
+        return x
+    raise TypeError("no JSON form for %r" % type(x))
+
+
+def sha_json(x):
+    """sha1 of the canonical JSON form of x: compares a whole spec field or launch op in 40 characters."""
+    return hashlib.sha1(json.dumps(jsonable(x), sort_keys=True).encode()).hexdigest()
+
+
+TRAINING_BUFFERS = ("rpn_acc", "rpn_precision", "rpn_recall", "rpn_metrics", "rpn_cls_loss", "rpn_loc_loss",
+                    "rpn_total_loss")
+
+
+def state_dict_json(sd):
+    """{"tensors": {key: [dtype, shape]}, "weights_sha1": sha1 over (key, dtype, shape, bytes) of every entry in key
+    order, the reference's training-metric buffers left out}."""
+    h = hashlib.sha1()
+    for k in sorted(sd):
+        if k.split(".")[0] not in TRAINING_BUFFERS:
+            h.update(json.dumps([k, digest(sd[k])]).encode())
+    return {"tensors": {k: [digest(v)["dtype"], list(v.shape)] for k, v in sd.items()}, "weights_sha1": h.hexdigest()}
+
+
+def load_json(name):
+    with open(os.path.join(GOLDEN_DIR, name)) as f:
+        return json.load(f)
+
+
+def detections_json(out):
+    """the detections of one frame (box3d_lidar / scores / label_preds) as exact JSON lists."""
+    return {k: np.asarray(out[k]).tolist() for k in ("box3d_lidar", "scores", "label_preds")}
+
+
+def voxels_json(res):
+    """digests of a voxelizer result (the network input, so a forward comparison starts from the same data)."""
+    return {k: digest(res[k]) for k in ("voxels", "coordinates", "num_points_per_voxel")}
 
 
 def cases():

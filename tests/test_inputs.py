@@ -1,6 +1,7 @@
 """On-GPU input path (SURVEY.md §8(f)1): NuScenes sweep merge and KITTI camera-FOV crop.
 CPU: the oracle restatement (oracle/py/inputs_ref.py) and the host-side calibration algebra (b2second.inputs) against
-the UNMODIFIED reference functions (container only).  GPU: the CUDA kernels against the oracle, bit for bit."""
+what the UNMODIFIED reference functions returned on the same inputs (tests/golden/reference_inputs.json).  GPU: the
+CUDA kernels against the oracle, bit for bit."""
 import os
 import sys
 
@@ -8,8 +9,9 @@ import numpy as np
 import pytest
 import torch
 
+import golden_util as gu
 from conftest import REPO
-from b2second import inputs, refcompat, synth
+from b2second import inputs, synth
 
 sys.path.insert(0, os.path.join(REPO, "oracle", "py"))
 import inputs_ref  # noqa: E402
@@ -56,52 +58,31 @@ def sweep_case(seed, n_sweeps=4, n=3000):
     return sweeps, rots, trans, lags
 
 
-needs_ref = pytest.mark.skipif(not refcompat.reference_available(), reason="reference tree not present")
+@pytest.fixture(scope="module")
+def ref_inputs():
+    """what the reference's own functions returned on the inputs below (tests/golden/make_dropin_golden.py)"""
+    return gu.load_json("reference_inputs.json")
 
 
-@needs_ref
-def test_crop_restatement_equals_reference_remove_outside_points(ref_env):
-    from second.core import box_np_ops
+def test_crop_restatement_equals_reference_remove_outside_points(ref_inputs):
+    """box_np_ops.remove_outside_points of the reference, on the same cloud and calibration."""
     P2, rect, Trv2c, shape = kitti_calib()
     pts = raw_kitti_cloud(0, 20000)
-    ref = box_np_ops.remove_outside_points(pts, rect, Trv2c, P2, shape)
+    assert gu.digest(pts) == ref_inputs["crop"]["points"], "synthetic cloud generator drifted"
     planes = inputs.frustum_planes(rect, Trv2c, P2, shape)
     got = inputs_ref.crop_convex_np(pts, planes)
     assert 0 < got.shape[0] < pts.shape[0] // 2 + 100
-    assert np.array_equal(ref, got)
+    assert gu.digest(got) == ref_inputs["crop"]["kept"]
 
 
-@needs_ref
-def test_sweep_merge_restatement_equals_reference_dataset_code(ref_env, tmp_path):
-    """run the reference's own NuScenesDataset.get_sensor_data on sweep files written to disk."""
-    import types
-    # external shims for modules the dataset file imports at top level but this code path never uses (the reference
-    # tree itself is untouched): scikit-image (kitti_common.py:9) and fire (nuscenes_dataset.py:10)
-    for name in ("skimage", "skimage.io", "fire"):
-        if name not in sys.modules:
-            try:
-                __import__(name)
-            except ImportError:
-                sys.modules[name] = types.ModuleType(name)
-    if not hasattr(sys.modules["skimage"], "io"):
-        sys.modules["skimage"].io = sys.modules["skimage.io"]
-    from second.data.nuscenes_dataset import NuScenesDataset
+def test_sweep_merge_restatement_equals_reference_dataset_code(ref_inputs):
+    """the reference's own NuScenesDataset.get_sensor_data on these sweeps written to disk."""
     sweeps, rots, trans, lags = sweep_case(1)
-    ts = 1.5e15
-    paths = []
-    for i, p in enumerate(sweeps):
-        f = tmp_path / ("s%d.bin" % i)
-        p.tofile(str(f))
-        paths.append(str(f))
-    info = {"token": "t", "lidar_path": paths[0], "timestamp": ts,
-            "sweeps": [{"lidar_path": paths[i], "timestamp": ts - lags[i] * 1e6, "sweep2lidar_rotation": rots[i],
-                        "sweep2lidar_translation": trans[i]} for i in range(1, len(sweeps))]}
-    ds = object.__new__(NuScenesDataset)
-    ds._nusc_infos = [info]
-    ref = ds.get_sensor_data(0)["lidar"]["points"]
+    assert [gu.digest(p) for p in sweeps] == ref_inputs["sweep_merge"]["sweeps"]
+    ts = ref_inputs["sweep_merge"]["timestamp"]
     true_lags = [0.0] + [ts / 1e6 - (ts - lags[i] * 1e6) / 1e6 for i in range(1, len(sweeps))]
     got = inputs_ref.merge_sweeps_np(sweeps, rots, trans, true_lags)
-    assert ref.shape == got.shape and np.array_equal(ref.astype(np.float32), got)
+    assert got.dtype == np.float32 and gu.digest(got) == ref_inputs["sweep_merge"]["merged"]
 
 
 @pytest.mark.gpu
