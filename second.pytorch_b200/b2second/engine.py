@@ -47,8 +47,9 @@ def ctypes_ptr(addr):
 
 
 class _Level:
-    """one active-site set: coordinates, device count, coordinate->row hash, row capacity."""
-    __slots__ = ("coors", "n_dev", "keys", "vals", "hcap", "cap", "shape")
+    """one active-site set: coordinates, device count, coordinate->row hash, row capacity.  `hashed`: the hash is
+    built every step (level 0 always; a strided conv's output only when some SubM rulebook probes it)."""
+    __slots__ = ("coors", "n_dev", "keys", "vals", "hcap", "cap", "shape", "hashed")
 
 
 class InferenceEngine:
@@ -101,6 +102,7 @@ class InferenceEngine:
         lv.cap = int(cap)
         lv.shape = [int(x) for x in shape]
         lv.hcap = _pow2_at_least(2 * lv.cap)
+        lv.hashed = True
         if with_storage:
             lv.coors = torch.zeros(lv.cap, 4, dtype=torch.int32, device=self.dev)
             lv.n_dev = torch.zeros(1, dtype=torch.int32, device=self.dev)
@@ -195,6 +197,7 @@ class InferenceEngine:
             if not lyr["subm"]:
                 lyr["want_hash"] = any(l["subm"] and l.get("build_rb") and l["in_level"] is lyr["out_level"]
                                        and not l.get("ranked") for l in self.layers)
+                lyr["out_level"].hashed = lyr["want_hash"]
         # once a layer runs on the tensor pipe all later ones must too (hi/lo planes flow forward)
         seen_tc = False
         for lyr in self.layers:
@@ -471,10 +474,12 @@ class InferenceEngine:
                                                       L.ptr(lin.vals), lin.hcap, L.ptr(lyr["rb"]["nbr"]),
                                                       L.ptr(lyr["rb"].get("row_mask")), st), "b2s_rulebook_subm")
                     else:
+                        # a level without a built hash passes none: its keys are uninitialised memory
                         L.check(lib.b2s_rulebook_conv(
                             L.ptr(lin.coors), L.ptr(lin.n_dev), lin.cap, self.B, L.i3(lin.shape), L.i3(lout.shape),
                             L.i3(lyr["kernel_size"]), L.i3(lyr["stride"]), L.i3(lyr["padding"]), L.i3(lyr["dilation"]),
-                            L.ptr(lin.keys), L.ptr(lin.vals), lin.hcap, L.ptr(lout.coors), L.ptr(lout.n_dev), lout.cap,
+                            L.ptr(lin.keys) if lin.hashed else None, L.ptr(lin.vals) if lin.hashed else None,
+                            lin.hcap, L.ptr(lout.coors), L.ptr(lout.n_dev), lout.cap,
                             L.ptr(lyr["rb"]["nbr"]), L.ptr(lout.keys) if lyr["want_hash"] else None,
                             L.ptr(lout.vals) if lyr["want_hash"] else None, lout.hcap,
                             L.ptr(self.rb_ws), self.rb_ws_bytes, L.ptr(lyr["rb"].get("row_mask")), L.ptr(self.status), st),

@@ -529,9 +529,11 @@ extern "C" int b2s_rulebook_conv(const int *coors_in, const int *num_in_dev, int
     B2S_LAUNCH_OK();
     k_scan_sums<<<1, kScanThreads, 0, stream>>>(w.chunk_sums, 0, w.nnz, num_out_dev, cap_out, status_dev);
     B2S_LAUNCH_OK();
-    static int use_scatter = -1;   // B2S_RB_SCATTER=0: neighbour table by hash probes from the output side (k_conv_nbr)
-    if (use_scatter < 0) { const char *e = getenv("B2S_RB_SCATTER"); use_scatter = (e && e[0] == '0') ? 0 : 1; }
-    if (!hash_keys_in) use_scatter = 1;
+    // B2S_RB_SCATTER=0: neighbour table by hash probes from the output side (k_conv_nbr), where an input hash exists.
+    // The environment is read once; the choice is made per call, so a call without an input hash never changes it.
+    static int env_scatter = -1;
+    if (env_scatter < 0) { const char *e = getenv("B2S_RB_SCATTER"); env_scatter = (e && e[0] == '0') ? 0 : 1; }
+    const int use_scatter = (env_scatter || !hash_keys_in) ? 1 : 0;
     k_conv_emit<<<bounded_grid(w.nwords < (1ll << 22) ? w.nwords : (1ll << 22), kThreads), kThreads, 0, stream>>>(
         w.bitmap, w.nz_word, w.nz_prefix, w.chunk_sums, w.nnz, g, cap_out, coors_out, use_scatter ? nbr : nullptr, w.wrow0);
     B2S_LAUNCH_OK();
