@@ -6,6 +6,8 @@ strides [1]) is: 6 x [Conv3x3 pad1 + BN + ReLU] -> deblock ConvTranspose2d(k=1,s
 heads.  Each becomes one b2s_conv2d_tc launch on NHWC halo-padded fp16 hi/lo planes; the three heads are one launch
 writing a packed 32-float record per pixel (box | cls | dir | pad) that b2s_decode_filter_strided reads.
 """
+import os
+
 import numpy as np
 import torch
 from torch import nn
@@ -103,6 +105,12 @@ def _conv_out(n, k, s, pad):
     return (n + 2 * pad - k) // s + 1
 
 
+def conv_v2_enabled():
+    """the switch the library's dispatch reads (conv_tc.cu, once per process): B2S_CONV_V2 starting with "0" sends the
+    3x3 stride-1 layers to k_conv_tc, which takes no tile lists."""
+    return not os.environ.get("B2S_CONV_V2", "").startswith("0")
+
+
 def plan_rpn(rpn, H, W, dry=False):
     """RPNV2 (second/pytorch/models/rpn.py:469-497 blocks, :264-299 deblocks, :386-420 heads) on an H x W BEV map ->
     {"buffers": {name: (h, w, c)}, "ops": [conv op dicts in execution order], "heads": {...}}.
@@ -111,6 +119,7 @@ def plan_rpn(rpn, H, W, dry=False):
     ConvTranspose2d; output channels are cut into slices of <= 128 (the kernel's n_pad) and `torch.cat` of the
     deblock outputs is a channel offset into the shared "cat" buffer."""
     bufs, ops = {}, []
+    use_v2 = conv_v2_enabled()
 
     def emit(kind, src, dst, w_t_co_ci, kh, kw, stride, pad, scale, shift, relu, hin, win, hg, wg, hout, wout,
              out_mul=1, off=(0, 0), dst_coff=0, planes=2, padded=True):
@@ -125,8 +134,8 @@ def plan_rpn(rpn, H, W, dry=False):
                  "dst_coff": dst_coff + c0, "planes": planes, "padded": padded,
                  "shift": None if shift is None else shift[c0:c1].float().contiguous(),
                  # the weights-stationary N=256 kernel takes this op (conv_tc.cu dispatch)
-                 "v2": (kh == 3 and kw == 3 and stride == 1 and pad == 1 and n_pad == 128 and planes == 2 and padded
-                        and out_mul == 1)}
+                 "v2": (use_v2 and kh == 3 and kw == 3 and stride == 1 and pad == 1 and n_pad == 128 and planes == 2
+                        and padded and out_mul == 1)}
             if not dry:
                 # weights pre-scaled by a power of two (exact), undone by the epilogue scale
                 wp = _pad_rows(w_t_co_ci[:, c0:c1].float(), n_pad)

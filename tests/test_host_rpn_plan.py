@@ -110,11 +110,9 @@ def bg_plan_numpy(occ, num_layers, tile=16):
         for dy in range(3):
             for dx in range(3):
                 out |= pad[:, dy:dy + H, dx:dx + W]
-        f = np.zeros((B, th, tw), np.int32)
-        for i in range(th):
-            for j in range(tw):
-                f[:, i, j] = out[:, i * tile:(i + 1) * tile, j * tile:(j + 1) * tile].any(axis=(1, 2))
-        flags.append(f)
+        # partial last tiles: the pixels past the image are False
+        full = np.pad(out, ((0, 0), (0, th * tile - H), (0, tw * tile - W)), constant_values=False)
+        flags.append(full.reshape(B, th, tile, tw, tile).any(axis=(2, 4)).astype(np.int32))
         cur = out
     return flags
 
@@ -169,6 +167,20 @@ def test_background_tiles_hold_the_empty_frame_response(name):
     inner = empty[0, :, 8:-8, 8:-8]
     assert float((inner - inner[:, :1, :1]).abs().max()) == 0.0
     assert float((empty[0, :, 0, 0] - inner[:, 0, 0]).abs().max()) > 0.0
+
+
+@pytest.mark.parametrize("switch,want", [(None, 6), ("1", 6), ("0", 0)])
+def test_conv_v2_switch_reaches_the_plan(monkeypatch, switch, want):
+    """B2S_CONV_V2=0 sends the 3x3 stride-1 layers to k_conv_tc, which refuses tile lists (conv_tc.cu): the plan must
+    then mark no op v2 and track no background layer, or the engine would pass lists the library rejects."""
+    if switch is None:
+        monkeypatch.delenv("B2S_CONV_V2", raising=False)
+    else:
+        monkeypatch.setenv("B2S_CONV_V2", switch)
+    net = models.build_network(config.get_config("car.fhd"), loader.oracle_spconv()).eval()
+    plan = tc.plan_rpn(net.rpn, 200, 176, dry=True)
+    assert sum(op["v2"] for op in plan["ops"]) == want
+    assert len(tc.background_layers(plan)) == want
 
 
 def test_fused_tail_is_taken_exactly_where_the_program_has_that_shape():
